@@ -31,6 +31,7 @@ L2_BYTES = 126e6
 IN_BYTES_PER_QP = 42 * 8 + 4     # x0[12] rot[9] foot[12] ref[9] fp64 + contact mask
 OUT_BYTES_PER_QP = 12 * 8 + 4    # f_body[12] fp64 + status
 ALG_BYTES_PER_QP = IN_BYTES_PER_QP + OUT_BYTES_PER_QP   # 440 B (SURVEY 8d)
+DUMP_BYTES = 60 * 1000 * 1000    # --dump-outputs: below 64 MB with the .npy headers
 
 
 def algorithmic_flops(N, ns_hist, fact_by_class):
@@ -250,6 +251,23 @@ def timed_steps(eng, dist, step, K, W):
     return dist_max(dist, eng.elapsed_ms(e0, e1)) / K
 
 
+def dump_outputs(out_dir, d, rank, world):
+    """what a caller of the timed path receives from one step -- forces [12, B] and status [B] of batch `d` -- as float64 .npy files,
+    so that two builds run with the same arguments can be compared output for output.  Above DUMP_BYTES (shared by the ranks) a
+    fixed, seeded sample of the QPs is written, with their indices in qp_index.npy.  Ranks other than 0 add _rank<r> to the names."""
+    f, status = d.download()
+    arrays = {"f_body": f.astype(np.float64), "status": status.astype(np.float64)}
+    B = status.shape[0]
+    keep_max = DUMP_BYTES // world // (14 * 8)        # f_body[12] + status + qp_index per sampled QP
+    if B * 13 * 8 > DUMP_BYTES // world:
+        keep = np.sort(np.random.default_rng(0).choice(B, keep_max, replace=False))
+        arrays = {"f_body": arrays["f_body"][:, keep], "status": arrays["status"][keep], "qp_index": keep.astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "_rank%d" % rank if rank else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), np.ascontiguousarray(a))
+
+
 def _status_hist(a1mpc, eng, d, B):
     st = np.zeros(B, dtype=np.int32)
     a1mpc._check(a1mpc.lib().a1mpc_memcpy_d2h(eng.h, st.ctypes.data, d.status, st.nbytes))
@@ -408,6 +426,7 @@ def main():
     ap.add_argument("--collect", default="auto", choices=["auto", "peer", "nccl"], help="final collect for --gpus > 1")
     ap.add_argument("--ring", type=int, default=0, help="number of distinct input batches (0: enough to exceed L2)")
     ap.add_argument("--no-subrecords", action="store_true", help="skip the config3 / config4 / config5 sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the forces and statuses of the last timed step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -480,6 +499,8 @@ def main():
     launches = eng.launches() - launches0
     ms = dist_max(dist, ms_local)
     value = n_gpus * B * K / (ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dev[(W + K - 1) % ring], rank, n_gpus)     # before the passes below overwrite the ring's outputs
 
     collect_ok = None
     if collect_fn is not None:

@@ -33,6 +33,12 @@ def load_ref_golden():
         return {k: z[k] for k in z.files}
 
 
+def load_ref_live():
+    """what the reference build returned on the inputs of the tests that compare with it (tests/golden/make_ref_live_golden.py)"""
+    with np.load(os.path.join(ROOT, "tests", "golden", "ref_live_v1.npz")) as z:
+        return {k: z[k] for k in z.files}
+
+
 def ref_cfg_kwargs(G, w):
     """keyword arguments (mass, inertia, q, r) of weight set w of the reference golden file, for O.make_config / a1mpc.default_config"""
     v = G["w%d" % w]

@@ -154,20 +154,20 @@ def test_neighbour_rows_oracle_sanity(O):
 
 def test_kinematics_oracle_is_pinned_to_the_reference(O):
     """golden vectors generated from the REFERENCE's own A1Kinematics::fk / jac (tests/golden/make_kin_golden.py, built by
-    `make -C oracle ref` where /root/reference exists); and, when that build is present, a fresh random comparison"""
-    from common import load_kin_golden
+    `make -C oracle ref`); and 500 random draws against what that build returned for them (tests/golden/ref_live_v1.npz)"""
+    from common import load_kin_golden, load_ref_live
     g = load_kin_golden()
     assert len(g["cases"]) >= 64
     for c in g["cases"]:
         p, J = O.leg_kinematics(c["q"], c["rho_opt"], c["rho_fix"])
         assert np.abs(p - np.array(c["p"])).max() <= 1e-14 and np.abs(J.reshape(9) - np.array(c["J"])).max() <= 1e-14
+    L = load_ref_live()
+    kin_p, kin_J = L["kin_p"], L["kin_J"]
     rng = np.random.default_rng(7)
-    if O.ref_leg_kinematics(np.zeros(3), np.zeros(3), np.ones(5)) is not None:
-        for _ in range(500):
-            q = rng.uniform(-2, 2, 3); ro = rng.normal(0, 0.05, 3); rf = rng.normal(0, 0.2, 5)
-            pr, Jr = O.ref_leg_kinematics(q, ro, rf)
-            p, J = O.leg_kinematics(q, ro, rf)
-            assert np.abs(p - pr).max() <= 1e-14 and np.abs(J - Jr).max() <= 1e-14
+    for k in range(500):
+        q = rng.uniform(-2, 2, 3); ro = rng.normal(0, 0.05, 3); rf = rng.normal(0, 0.2, 5)
+        p, J = O.leg_kinematics(q, ro, rf)
+        assert np.abs(p - kin_p[k]).max() <= 1e-14 and np.abs(J - kin_J[k]).max() <= 1e-14
 
 
 def test_ekf_oracle_sanity(O):
