@@ -18,7 +18,7 @@ all: $(LIB) oracle host
 $(OBJ):
 	mkdir -p $(OBJ)
 
-$(OBJ)/%.o: $(SRC)/%.cu $(SRC)/a1mpc_device.cuh $(SRC)/a1mpc_sched.cuh $(SRC)/a1mpc_estim.cuh $(SRC)/a1mpc_misc.cuh $(SRC)/a1mpc_solve_body.inc $(SRC)/a1mpc_solve_n10.cu $(SRC)/a1mpc_internal.h include/a1mpc.h | $(OBJ)
+$(OBJ)/%.o: $(SRC)/%.cu $(SRC)/a1mpc_device.cuh $(SRC)/a1mpc_sched.cuh $(SRC)/a1mpc_estim.cuh $(SRC)/a1mpc_misc.cuh $(SRC)/a1mpc_solve_body.inc $(SRC)/a1mpc_sched2_body.inc $(SRC)/a1mpc_solve_n10.cu $(SRC)/a1mpc_internal.h include/a1mpc.h | $(OBJ)
 	$(NVCC) $(NVFLAGS) -c $< -o $@ 2> $(OBJ)/$*.ptxas.log || (cat $(OBJ)/$*.ptxas.log; false)
 
 $(OBJ)/%.o: $(SRC)/%.cpp include/a1mpc.h | $(OBJ)

@@ -17,7 +17,7 @@ STATUS_OPTIMAL, STATUS_IPM_ONLY, STATUS_MAXITER, STATUS_NUMERICAL, STATUS_NO_CON
 
 EXPORTS = [
     "a1mpc_default_config", "a1mpc_create", "a1mpc_destroy", "a1mpc_last_error", "a1mpc_device_count",
-    "a1mpc_solve_batch", "a1mpc_warm_bytes", "a1mpc_warm_reset", "a1mpc_solve_batch_warm", "a1mpc_solve_batch_ext", "a1mpc_build_qp_batch", "a1mpc_qp_mats_batch", "a1mpc_solve_dense_batch",
+    "a1mpc_solve_batch", "a1mpc_warm_bytes", "a1mpc_warm_reset", "a1mpc_solve_batch_warm", "a1mpc_solve_batch_ext", "a1mpc_solve_batch_ext_warm", "a1mpc_build_qp_batch", "a1mpc_qp_mats_batch", "a1mpc_solve_dense_batch",
     "a1mpc_grf_qp_batch", "a1mpc_joint_torques_batch", "a1mpc_leg_kinematics_batch", "a1mpc_ekf_bytes", "a1mpc_ekf_init_batch", "a1mpc_ekf_update_batch", "a1mpc_update_plan_batch", "a1mpc_device_alloc", "a1mpc_device_free", "a1mpc_host_alloc", "a1mpc_host_free",
     "a1mpc_memcpy_h2d", "a1mpc_memcpy_d2h", "a1mpc_sync", "a1mpc_event_create", "a1mpc_event_destroy",
     "a1mpc_event_record", "a1mpc_event_elapsed_ms", "a1mpc_launch_count", "a1mpc_measure_fp64_peak",
@@ -107,6 +107,7 @@ def lib():
         l.a1mpc_ekf_init_batch.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
         l.a1mpc_ekf_update_batch.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_double, C.c_int] + [C.c_void_p] * 11
         l.a1mpc_solve_batch_ext.argtypes = [C.c_void_p, C.c_int, C.POINTER(Inputs), C.POINTER(InputsExt), C.POINTER(Outputs)]
+        l.a1mpc_solve_batch_ext_warm.argtypes = [C.c_void_p, C.c_int, C.POINTER(Inputs), C.POINTER(InputsExt), C.POINTER(Outputs), C.c_void_p, C.c_int]
         l.a1mpc_gen_schedule.argtypes = [C.c_int, C.c_uint64, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
         l.a1mpc_build_qp_batch.argtypes = [C.c_void_p, C.c_int, C.POINTER(Inputs), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         l.a1mpc_qp_mats_batch.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 6
@@ -275,6 +276,23 @@ class Engine:
         ext = InputsExt(_p(sc), _p(nm))
         out = Outputs(_p(f), _p(status), _p(iters), _p(u), B)
         _check(lib().a1mpc_solve_batch_ext(self.h, B, C.byref(inp), C.byref(ext), C.byref(out)))
+        return (f, status, iters, u) if want_u else (f, status, iters)
+
+    def solve_ext_warm(self, st, warm, sched=None, normals=None, shift=1, want_u=False):
+        """a1mpc_solve_batch_ext_warm: solve_ext with the warm start of solve_warm (`warm` from warm_alloc, updated in place on
+        the device); shift = 1 for schedules that advance one step per tick (update_plan)"""
+        B = st["x0"].shape[1]
+        N = self.cfg.horizon
+        ft = self.ftype
+        a = {k: np.ascontiguousarray(st[k], dtype=(np.uint32 if k == "contact" else ft)) for k in ("x0", "rot", "foot", "ref", "contact")}
+        sc = np.ascontiguousarray(sched, dtype=np.uint32) if sched is not None else None
+        nm = np.ascontiguousarray(normals, dtype=ft) if normals is not None else None
+        f = np.zeros((12, B), dtype=ft); status = np.zeros(B, dtype=np.int32); iters = np.zeros(B, dtype=np.int32)
+        u = np.zeros((12 * N, B), dtype=ft) if want_u else None
+        inp = Inputs(_p(a["x0"]), _p(a["rot"]), _p(a["foot"]), _p(a["ref"]), _p(a["contact"]), B)
+        ext = InputsExt(_p(sc), _p(nm))
+        out = Outputs(_p(f), _p(status), _p(iters), _p(u), B)
+        _check(lib().a1mpc_solve_batch_ext_warm(self.h, B, C.byref(inp), C.byref(ext), C.byref(out), warm, int(shift)))
         return (f, status, iters, u) if want_u else (f, status, iters)
 
     def solve_ptrs(self, B, inp, out):

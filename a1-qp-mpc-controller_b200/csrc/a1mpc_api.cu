@@ -45,6 +45,7 @@ struct a1mpc_handle {
   a1mpc::ClassLaunch cls[5];  // index = number of stance feet
   a1mpc::ClassLaunch cls_ext;  // extended path (config 4)
   a1mpc::ClassLaunch cls_sched2;   // its compacted two-feet-per-step class (N = 10; A1MPC_EXT_COMPACT=0 disables it)
+  a1mpc::ClassLaunch cls_ext_warm, cls_sched2_warm;   // the same two with the warm start (a1mpc_solve_batch_ext_warm)
   bool ext_compact = false;
   double* d_rec_ext = nullptr;
   size_t cap_ext = 0;
@@ -303,13 +304,13 @@ int a1mpc_create(a1mpc_handle** out, const a1mpc_config* cfg, int device) {
   {
     cudaError_t e = (cfg->horizon == 10) ? fused_setup_n10(h->sm_count, h->cls) : fused_setup_n20(h->sm_count, h->cls);
     if (e != cudaSuccess) return bail(fail(A1MPC_ECUDA, std::string("kernel setup: ") + cudaGetErrorString(e)));
-    e = ext_setup(cfg->horizon, h->sm_count, h->cls_ext);
+    e = ext_setup(cfg->horizon, h->sm_count, h->cls_ext, h->cls_ext_warm);
     if (e != cudaSuccess) return bail(fail(A1MPC_ECUDA, std::string("ext kernel setup: ") + cudaGetErrorString(e)));
     {   // schedules with two stance feet in every step run on the compact direct kernel (a1mpc_sched.cuh): 2.5 M instead of 1.5 M
         // QPs/s end to end on a B200 at B = 16384 (profiles/r02a_call1_*.txt).  A1MPC_EXT_COMPACT=0 keeps everything on the general kernel (A/B).
       const char* ev = std::getenv("A1MPC_EXT_COMPACT");
       if (!(ev && ev[0] == '0') && cfg->horizon == 10) {
-        e = sched2_setup(h->sm_count, h->cls_sched2);
+        e = sched2_setup(h->sm_count, h->cls_sched2, h->cls_sched2_warm);
         if (e != cudaSuccess) return bail(fail(A1MPC_ECUDA, std::string("compact ext kernel setup: ") + cudaGetErrorString(e)));
         h->ext_compact = true;
       }
@@ -409,9 +410,10 @@ int a1mpc_solve_batch_warm(a1mpc_handle* h, int B, const a1mpc_inputs* in, const
   return solve_batch_impl(h, B, in, out, static_cast<uint32_t*>(warm), shift);
 }
 
-int a1mpc_solve_batch_ext(a1mpc_handle* h, int B, const a1mpc_inputs* in, const a1mpc_inputs_ext* ext, const a1mpc_outputs* out) {
-  if (!h || !in || !out) return fail(A1MPC_EINVAL, "null argument");
-  if (!ext || (!ext->contact_sched && !ext->normals)) return a1mpc_solve_batch(h, B, in, out);
+// the extended call, cold (warm == nullptr) or warm-started: argument checks, device mirrors and packing are shared, only
+// the solve launches differ.  The caller has checked h, in, out and that ext carries a schedule or normals.
+static int solve_ext_impl(a1mpc_handle* h, int B, const a1mpc_inputs* in, const a1mpc_inputs_ext* ext, const a1mpc_outputs* out, uint32_t* warm,
+                          int shift) {
   if (B <= 0) return fail(A1MPC_EINVAL, "B must be positive");
   if (!in->x0 || !in->rot || !in->foot || !in->ref || !in->contact || !out->f_body || !out->status) return fail(A1MPC_EINVAL, "null input/output array");
   if (in->ld < (size_t)B || out->ld < (size_t)B) return fail(A1MPC_EINVAL, "ld < B");
@@ -471,15 +473,21 @@ int a1mpc_solve_batch_ext(a1mpc_handle* h, int B, const a1mpc_inputs* in, const 
   }
   attach_peers(h, -1, dout);   // the fused collect is wired to a1mpc_solve_batch / _warm only
   CK(cudaMemsetAsync(h->d_count, 0, 16 * sizeof(int), h->stream));
+  const ClassLaunch& cls_ext = warm ? h->cls_ext_warm : h->cls_ext;
   if (h->ext_compact && dsched) {
     pack_ext2_kernel<<<(B + 127) / 128, 128, 0, h->stream>>>(di, dsched, dnorm, B, h->d_rec_ext, (int)h->cap_ext, h->d_count, dout, N);
-    ext_launch(N, h->cls_ext, h->stream, B, h->P, h->d_rec_ext, h->d_count, dout);
-    sched2_launch(h->cls_sched2, h->stream, B, h->P, h->d_rec_ext + h->cap_ext * REC_EXT_DOUBLES, h->d_count, dout);
+    ext_launch(N, cls_ext, h->stream, B, h->P, h->d_rec_ext, h->d_count, dout, warm, shift);
+    sched2_launch(warm ? h->cls_sched2_warm : h->cls_sched2, h->stream, B, h->P, h->d_rec_ext + h->cap_ext * REC_EXT_DOUBLES, h->d_count, dout,
+                  warm, shift);
     h->launches += 3;
   } else {
     pack_ext_kernel<<<(B + 127) / 128, 128, 0, h->stream>>>(di, dsched, dnorm, B, h->d_rec_ext, h->d_count, dout, N);
-    ext_launch(N, h->cls_ext, h->stream, B, h->P, h->d_rec_ext, h->d_count, dout);
+    ext_launch(N, cls_ext, h->stream, B, h->P, h->d_rec_ext, h->d_count, dout, warm, shift);
     h->launches += 2;
+  }
+  if (warm) {
+    warm_clear_idle_kernel<<<(B + 127) / 128, 128, 0, h->stream>>>(di.contact, dsched, di.ld, B, N, warm);
+    h->launches++;
   }
   CK(cudaGetLastError());
   if (!dev) {
@@ -491,6 +499,22 @@ int a1mpc_solve_batch_ext(a1mpc_handle* h, int B, const a1mpc_inputs* in, const 
     CK(cudaStreamSynchronize(h->stream));
   }
   return A1MPC_OK;
+}
+
+int a1mpc_solve_batch_ext(a1mpc_handle* h, int B, const a1mpc_inputs* in, const a1mpc_inputs_ext* ext, const a1mpc_outputs* out) {
+  if (!h || !in || !out) return fail(A1MPC_EINVAL, "null argument");
+  if (!ext || (!ext->contact_sched && !ext->normals)) return a1mpc_solve_batch(h, B, in, out);
+  return solve_ext_impl(h, B, in, ext, out, nullptr, 0);
+}
+
+int a1mpc_solve_batch_ext_warm(a1mpc_handle* h, int B, const a1mpc_inputs* in, const a1mpc_inputs_ext* ext, const a1mpc_outputs* out, void* warm,
+                               int shift) {
+  if (!h || !in || !out || !warm) return fail(A1MPC_EINVAL, "null argument");
+  if (!ext || (!ext->contact_sched && !ext->normals)) return a1mpc_solve_batch_warm(h, B, in, out, warm, shift);
+  if (shift < 0 || shift > h->cfg.horizon) return fail(A1MPC_EINVAL, "shift out of range");
+  CK(cudaSetDevice(h->device));
+  if (!is_device_ptr(warm)) return fail(A1MPC_EINVAL, "warm must be device memory (a1mpc_device_alloc)");
+  return solve_ext_impl(h, B, in, ext, out, static_cast<uint32_t*>(warm), shift);
 }
 
 int a1mpc_build_qp_batch(a1mpc_handle* h, int B, const a1mpc_inputs* in, double* H, double* g, double* lb, double* ub) {

@@ -20,12 +20,15 @@ void fused_launch_n20(int ns, const ClassLaunch& c, cudaStream_t st, int B, cons
 // warm-started variant of the N = 10 classes (a1mpc_solve_batch_warm); set up by fused_setup_n10
 void fused_launch_n10_warm(int ns, const ClassLaunch& c, cudaStream_t st, int B, const DevParams& P, const double* rec, const int* count,
                            const DevOutputs& out, uint32_t* warm, int shift);
-// extended path (per-step contact schedules + terrain normals), a1mpc_solve_ext.cu
-cudaError_t ext_setup(int horizon, int sm_count, ClassLaunch& c);
-void ext_launch(int horizon, const ClassLaunch& c, cudaStream_t st, int B, const DevParams& P, const double* rec, const int* count, const DevOutputs& out);
-// compacted two-stance-feet-per-step class of the extended path (a1mpc_sched.cuh; opt-in, N = 10)
-cudaError_t sched2_setup(int sm_count, ClassLaunch& c);
-void sched2_launch(const ClassLaunch& c, cudaStream_t st, int B, const DevParams& P, const double* rec, const int* count, const DevOutputs& out);
+// extended path (per-step contact schedules + terrain normals), a1mpc_solve_ext.cu.  `cw` / warm != nullptr: the warm-started
+// kernels of a1mpc_solve_batch_ext_warm (their own occupancy, launched with the ClassLaunch that setup filled for them)
+cudaError_t ext_setup(int horizon, int sm_count, ClassLaunch& c, ClassLaunch& cw);
+void ext_launch(int horizon, const ClassLaunch& c, cudaStream_t st, int B, const DevParams& P, const double* rec, const int* count, const DevOutputs& out,
+                uint32_t* warm = nullptr, int shift = 0);
+// compacted two-stance-feet-per-step class of the extended path (a1mpc_sched.cuh; N = 10)
+cudaError_t sched2_setup(int sm_count, ClassLaunch& c, ClassLaunch& cw);
+void sched2_launch(const ClassLaunch& c, cudaStream_t st, int B, const DevParams& P, const double* rec, const int* count, const DevOutputs& out,
+                   uint32_t* warm = nullptr, int shift = 0);
 cudaError_t build_dense_launch(const DevParams& P, const DevInputs& in, int B, double* H, double* g, double* lb, double* ub, cudaStream_t st);
 
 // QP-major side entry points (a1mpc_dense.cu)

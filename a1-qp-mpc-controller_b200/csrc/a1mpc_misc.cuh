@@ -133,6 +133,17 @@ __global__ void pack_ext2_kernel(DevInputs in, const uint32_t* __restrict__ sche
   }
 }
 
+// a1mpc_solve_batch_ext_warm: a robot with no foot in contact anywhere in the horizon never reaches a solve kernel (the pack
+// kernels answer NO_CONTACT); its slot is marked "no guess" here, as the solve kernels do for every result that is not OPTIMAL
+__global__ void warm_clear_idle_kernel(const uint32_t* __restrict__ contact, const uint32_t* __restrict__ sched, size_t ld, int B, int horizon,
+                                       uint32_t* __restrict__ warm) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  uint32_t any = 0u;
+  for (int st = 0; st < horizon; ++st) any |= (sched ? sched[(size_t)st * ld + b] : contact[b]) & 15u;
+  if (any == 0u) warm[(size_t)b * (WARM_HDR + 4 * horizon)] = 0u;
+}
+
 // Classes whose factor does not fit in shared memory (N=20 with four stance feet in fp64):
 // reported, never silently approximated.
 __global__ void unsupported_kernel(const double* __restrict__ rec, const int* __restrict__ count, int cls, DevOutputs out, int horizon) {

@@ -4,7 +4,7 @@
 // the absent foot-steps; this one eliminates them: H_compact = Sel' (T0 (x) G0 + T1 (x) G1 + 2R) Sel with the full 12 x 12 Gram
 // blocks and a (step, leg) selection, solved by the direct 64 x 64 tensor-core core like the trot class.
 // OPT-IN this round (A1MPC_EXT_COMPACT=1 in the environment of a1mpc_create): validated on the CPU emulator only.
-// Include from a1mpc_solve_ext.cu and tests/emu.
+// Include from a1mpc_solve_ext.cu and tests/emu (the kernel body is a1mpc_sched2_body.inc).
 #pragma once
 #include "a1mpc_device.cuh"
 
@@ -116,119 +116,19 @@ struct SchedHess {
 template <int N, int WPC>
 __global__ void __launch_bounds__(32 * WPC) solve_kernel_sched2(const __grid_constant__ DevParams P, const double* __restrict__ rec,
                                                                 const int* __restrict__ count, DevOutputs out) {
-  using G = Geo<2, N, 0>;
-  using SG = SchedGeo<N>;
-  static_assert(G::TW == 1, "the compacted schedule kernel is written for one warp per QP (N = 10)");
-  A1MPC_DYN_SMEM(smem);
-  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  for (int e = threadIdx.x; e < N * N; e += blockDim.x) {
-    const int a = e / N, b = e - a * N, m = a > b ? a : b;
-    smem[e] = (double)(N - m);
-    int t1 = 0;
-    for (int i = m; i < N; ++i) t1 += (i - a) * (i - b);
-    smem[N * N + e] = (double)t1;
-  }
-  double* base = smem + G::TAB_DOUBLES + wib * SG::WARP_DOUBLES;
-  Ctx<2, N, 0> c(base, smem, lane);
-  double* xs = base + G::WARP_DOUBLES;
-  int* legmap = reinterpret_cast<int*>(xs + SG::X_LEG);
-  SchedHess<N> hp;
-  hp.legmap = legmap; hp.vinf = xs + SG::X_VIN; hp.voutf = xs + SG::X_VOUT;
-  hp.cf.lane = lane; hp.cf.tid = lane; hp.cf.wit = 0; hp.cf.barid = 0; hp.cf.rec = c.rec; hp.cf.L = c.L; hp.cf.T0 = c.T0; hp.cf.T1 = c.T1;
-  hp.cf.g = xs + SG::X_G; hp.cf.G0 = xs + SG::X_G0; hp.cf.G1 = xs + SG::X_G1; hp.cf.R2 = xs + SG::X_R2;
-  hp.cf.vp0 = xs + SG::X_VP0; hp.cf.vp1 = xs + SG::X_VP1;
-  hp.cf.vu = hp.cf.vrhs = hp.cf.vtmp = hp.cf.vy = nullptr; hp.cf.D = nullptr; hp.cf.zinfo = nullptr; hp.cf.exist = nullptr;
-  hp.cf.bar = nullptr; hp.cf.wx = nullptr; hp.cf.base_ = nullptr;
-  if (lane == 0) mbar_init(c.bar, 1);
-  if (A1MPC_RV && WPC > 1 && threadIdx.x == 0) mbar_init(smem + 2 * N * N, WPC);
-  __syncthreads();
-  const int nq = count[6];
-  // QP q -> warp q % WPC of CTA q / WPC: a class with few QPs fills few CTAs completely and leaves the other SMs to the classes that
-  // run concurrently on their own streams.  (Spreading one QP per CTA first was measured in round 2: a 4-stance CTA reserves its
-  // four warps' shared memory and registers whether or not they have work, the trot class lost 2/3 of the SMs to 102 QPs and took
-  // 0.43 instead of 0.25 ms at B = 1024, while the 4-stance kernel itself did not get faster -- its time is the slowest QP's
-  // factorisation count times a per-factorisation latency that one warp per scheduler already has to itself.)
-  const int gw = blockIdx.x * WPC + wib, nw = gridDim.x * WPC;
-  int* const head = const_cast<int*>(count) + 8 + 6;   // queue counter of this class (next_qp)
-  uint32_t parity = 0;
-#pragma unroll 1
-  for (int q = gw; q < nq; q = next_qp(c, head, q, nw)) {
-    if (lane == 0) tma_load_record(c.rec, rec + (size_t)q * REC_EXT_DOUBLES, c.bar, REC_EXT_DOUBLES * 8);
-    mbar_wait(c.bar, parity);
-    parity ^= 1u;
-    const int b = __double2loint(c.rec[42]);
-    const unsigned long long s0 = (unsigned long long)__double_as_longlong(c.rec[44]), s1 = (unsigned long long)__double_as_longlong(c.rec[45]);
-    // the two stance legs of every step, ascending
-    if (lane < N) {
-      const unsigned bits = (lane < 16) ? (unsigned)((s0 >> (4 * lane)) & 15ull) : (unsigned)((s1 >> (4 * (lane - 16))) & 15ull);
-      const int l0 = __ffs((int)bits) - 1;
-      const int l1 = __ffs((int)(bits & (bits - 1u))) - 1;
-      legmap[2 * lane] = l0;
-      legmap[2 * lane + 1] = l1;
-    }
-    bool bad = false;
-    for (int k = lane; k < 42; k += 32) bad = bad || !(fabs(c.rec[k]) < 1e300);
-    if (lane < 12) bad = bad || !(fabs(c.rec[46 + lane]) < 1e300);
-    bad = __any_sync(0xffffffffu, bad);
-    int status, iters = 0;
-    if (bad) {
-      status = A1MPC_STATUS_NUMERICAL;
-      for (int i = lane; i < G::NPAD; i += 32) c.vy[i] = 0.0;
-      __syncwarp();
-    } else {
-      const int all_legs[4] = {0, 1, 2, 3};
-      build_qp<4, N, 0, true>(hp.cf, P, all_legs);        // full-leg g, G0, G1, R2 (terrain frames included); scratch in c.L
-      for (int i = lane; i < G::NV; i += 32) {
-        const int k = i / 3, a = i - 3 * k;
-        c.g[i] = hp.cf.g[12 * (k >> 1) + 3 * legmap[k] + a];
-      }
-      __syncwarp();
-      fill_padding<2, N, 0>(c);
-      status = solve_qp<2, N, 0, SchedHess<N>, DirectLS<2, N, SchedHess<N>>>(c, hp, P, iters);
-    }
-    // outputs: legs in stance in the FIRST step carry a force; terrain frame -> world -> body (R^T)
-    double f[3] = {0.0, 0.0, 0.0};
-    if (lane < 4) {
-      int k0 = -1;
-      if (legmap[0] == lane) k0 = 0;
-      if (legmap[1] == lane) k0 = 1;
-      if (k0 >= 0 && !bad) {   // bad inputs: zero forces, nothing is multiplied with the poisoned record
-        const double ux = c.vy[3 * k0] * FSCALE, uy = c.vy[3 * k0 + 1] * FSCALE, uz = c.vy[3 * k0 + 2] * FSCALE;
-        double e0[3], e1[3], e2[3];
-        terrain_col(c.rec + 46 + 3 * lane, 0, e0); terrain_col(c.rec + 46 + 3 * lane, 1, e1); terrain_col(c.rec + 46 + 3 * lane, 2, e2);
-        const double wx_ = e0[0] * ux + e1[0] * uy + e2[0] * uz, wy_ = e0[1] * ux + e1[1] * uy + e2[1] * uz, wz_ = e0[2] * ux + e1[2] * uy + e2[2] * uz;
-#pragma unroll
-        for (int a = 0; a < 3; ++a) f[a] = c.rec[12 + a] * wx_ + c.rec[15 + a] * wy_ + c.rec[18 + a] * wz_;
-      }
-    }
-    st_forces(out, b, f, lane, c.vtmp);
-    if (lane == 0) {
-      out.status[b] = status;
-      if (out.iters) out.iters[b] = iters;
-    }
-    if (out.u_full) {
-      for (int e = lane; e < 12 * N; e += 32) {
-        const int st = e / 12, r = e - 12 * st, leg = r / 3, a = r - 3 * leg;
-        double v = 0.0;
-        int k = -1;
-        if (legmap[2 * st] == leg) k = 2 * st;
-        if (legmap[2 * st + 1] == leg) k = 2 * st + 1;
-        if (k >= 0 && !bad) {
-          double col[3], acc = 0.0;
-#pragma unroll
-          for (int bb = 0; bb < 3; ++bb) { terrain_col(c.rec + 46 + 3 * leg, bb, col); acc = fma(col[a], c.vy[3 * k + bb], acc); }
-          v = acc * FSCALE;
-        }
-        st_out(out.u_full, (size_t)e * out.ld + b, v, out.f32);
-      }
-    }
-    __syncwarp();
-    fence_proxy_async();
-  }
-  if (A1MPC_RV && WPC > 1) {
-    __syncwarp();
-    if (lane == 0) rv_drop(smem + 2 * N * N);
-  }
+  constexpr bool WARM = false;
+  uint32_t* const warm = nullptr;
+  const int shift = 0;
+#include "a1mpc_sched2_body.inc"
+}
+
+// the same kernel with the device-resident warm start (a1mpc_solve_batch_ext_warm; the slot format of WARM_HDR)
+template <int N, int WPC>
+__global__ void __launch_bounds__(32 * WPC) solve_kernel_sched2_warm(const __grid_constant__ DevParams P, const double* __restrict__ rec,
+                                                                     const int* __restrict__ count, DevOutputs out, uint32_t* __restrict__ warm,
+                                                                     int shift) {
+  constexpr bool WARM = true;
+#include "a1mpc_sched2_body.inc"
 }
 
 }  // namespace a1mpc

@@ -60,8 +60,9 @@ typedef struct a1mpc_handle a1mpc_handle;
  *   max_iter, tol    solver controls; 0 selects the defaults (40, 1e-9 switch-over mu)
  *   precision        64: every array of the boundary is fp64 (the reference's arithmetic type).
  *                    32: BASELINE config 3's "fp32" -- the floating-point arrays of the HOT-PATH boundary (a1mpc_solve_batch,
- *                        a1mpc_solve_batch_warm, a1mpc_solve_batch_ext: x0, rot, foot, ref, normals in; f_body, u_full out) hold
- *                        float instead of double, 224 instead of 440 bytes per QP; they are declared `double*` below and
+ *                        a1mpc_solve_batch_warm, a1mpc_solve_batch_ext, a1mpc_solve_batch_ext_warm: x0, rot, foot, ref, normals
+ *                        in; f_body, u_full out) hold float instead of double, 224 instead of 440 bytes per QP; they are
+ *                        declared `double*` below and
  *                        reinterpreted.  The arithmetic in between stays fp64 with the in-kernel KKT certificate: the reduced
  *                        systems have condition numbers of 1e5 (N=10) .. 1e6 (N=20), an fp32 factorisation cannot certify
  *                        1e-4 N, and the only fp32-input tensor-core MMA (tf32, 10-bit mantissa) breaks down on 85 % of the
@@ -160,6 +161,20 @@ typedef struct a1mpc_inputs_ext {
   const double*   normals;
 } a1mpc_inputs_ext;
 int  a1mpc_solve_batch_ext(a1mpc_handle* h, int B, const a1mpc_inputs* in, const a1mpc_inputs_ext* ext, const a1mpc_outputs* out);
+
+/* ---- warm start across control ticks for the extended call ---------------------------------------------------------
+ * a1mpc_solve_batch_ext with the device-resident warm start of a1mpc_solve_batch_warm: the same arguments, host / device
+ * rules, precision and outputs as a1mpc_solve_batch_ext, and `warm` / `shift` as for a1mpc_solve_batch_warm (same buffer
+ * format, a1mpc_warm_bytes / a1mpc_warm_reset; a slot written by either warm call may be read by the other).  Horizons 10
+ * and 20.  ext NULL or without schedule and normals: exactly a1mpc_solve_batch_warm.
+ * Guesses are per foot-step, not per robot: a change of stance feet does not force a cold start.  Foot-step (s, leg) starts
+ * from the face stored at (min(s + shift, N - 1), leg); a foot-step that is not in contact gets the swing face whatever the
+ * slot holds.  Only OPTIMAL results store faces; NUMERICAL, NO_CONTACT and uncertified robots store "no guess".
+ *   shift  1 is the natural setting with a1mpc_update_plan_batch, which advances every schedule by one horizon step per tick
+ *          (step st of the plan is the gait at counter + st * speed); a1mpc_solve_batch_warm's compute_grf-style 0 applies to a
+ *          pattern that is re-posed every tick.  Any shift gives the same optimum; a misaligned one only costs hits. */
+int  a1mpc_solve_batch_ext_warm(a1mpc_handle* h, int B, const a1mpc_inputs* in, const a1mpc_inputs_ext* ext, const a1mpc_outputs* out,
+                                void* warm, int shift);
 
 /* ---- ConvexMpc members, for parity with the reference class (ConvexMpc.h:87-93) ----------- */
 /* Dense QP data exactly as ConvexMpc::calculate_qp_mats leaves it after compute_grf drove it

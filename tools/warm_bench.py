@@ -1,6 +1,11 @@
 """dev tool: closed-loop throughput of the device-resident warm start (a1mpc_solve_batch_warm) next to the cold path.
 A ring of T consecutive control ticks (state advanced by dt plus a random walk of sensor-level noise) is uploaded once; the
-timed loop walks the ring.  Not part of bench.py's contract (that measures independent QPs, i.e. the cold path)."""
+timed loop walks the ring.  Not part of bench.py's contract (that measures independent QPs, i.e. the cold path).
+
+    python tools/warm_bench.py [B] [noise]      constant contact pattern (a1mpc_solve_batch / _warm, shift 0)
+    python tools/warm_bench.py --ext [B ...]    scheduled ticks: a1mpc_solve_batch_ext / _ext_warm (shift 1) with per-step
+                                                schedules that advance one step per tick and terrain normals, at noise 0.03
+                                                and 0.1, next to the constant-pattern pair on the same states"""
 import ctypes as C
 import os
 import sys
@@ -10,6 +15,12 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "a1-qp-mpc-controller_b200")); sys.path.insert(0, ROOT)
 import a1mpc
+
+if "--ext" in sys.argv:
+    sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+    import warm_bench_ext
+    warm_bench_ext.main([int(a) for a in sys.argv[1:] if a != "--ext"] or [1024, 16384])
+    sys.exit(0)
 
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 1024
 noise = float(sys.argv[2]) if len(sys.argv) > 2 else 0.1
